@@ -2,7 +2,7 @@
 """bench.py -- end-to-end frames/s of the per-frame ADAS path (YOLOv8l + UFLDv2-CULane-ResNet34 + ByteTrack) on
 synthetic 1280x720 frames, one process per GPU.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch 8] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch 8] [--impl b200|reference] [--dump-outputs DIR]
 
 A "step" = one batch of `--batch` consecutive frames of one stream through the whole hot path:
     frames -> [letterbox + YOLOv8l + DFL decode + candidate select + reference NMS]  (adas_yolo_detect)
@@ -70,6 +70,55 @@ def build_plans(seed: int = 0):
             os.replace(path + f".{os.getpid()}.tmp", path)
         out[kind] = (path, W.state_dict, pb)
     return out
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def _step_arrays(r, frames) -> dict:
+    f = np.asarray(frames)
+    counts, npts = np.asarray(r.counts)[f], np.asarray(r.lane_npts)[f]
+    det = np.arange(r.boxes.shape[1])[None, :] < counts[:, None]                   # [F, max_det]: rows past the count are unset
+    pts = np.arange(r.lane_pts.shape[2])[None, None, :] < npts[:, :, None]        # [F, 4, max_pts]
+    recs = [r.tracks[i] for i in f.tolist()]
+    cols = [np.concatenate([t[n].reshape(len(t), int(np.prod(t.dtype[n].shape))).astype(np.float64) for n in t.dtype.names], 1)
+            for t in recs]
+    return {
+        "frame_index": f.astype(np.float64),
+        "det_boxes": np.where(det[..., None], r.boxes[f], 0).astype(np.float32),
+        "det_scores": np.where(det, r.scores[f], 0).astype(np.float32),
+        "det_class_ids": np.where(det, r.class_ids[f], -1).astype(np.float64),
+        "det_cand_index": np.where(det, r.cand_index[f], -1).astype(np.float64),
+        "det_counts": counts.astype(np.float64),
+        "det_n_candidates": np.asarray(r.n_candidates)[f].astype(np.float64),
+        "lane_pts": np.where(pts[..., None], r.lane_pts[f], 0).astype(np.float64),
+        "lane_npts": npts.astype(np.float64),
+        "lane_status": np.asarray(r.lane_status)[f].astype(np.float64),
+        "track_counts": np.array([len(t) for t in recs], np.float64),
+        "tracks": np.concatenate(cols),
+    }
+
+
+def dump_outputs(r, out_dir: str, limit: int = DUMP_LIMIT) -> dict:
+    """Write what one pipeline step handed its caller as out_dir/<name>.npy (float32 / float64) so that two builds can be
+    compared output for output: detections (xywh boxes, scores, class ids, candidate indices, per-frame counts), lanes (points,
+    counts, status) and the tracker's records of every frame, concatenated in frame order (`track_counts` rows per frame; columns
+    are the fields of adas_b200._capi.TRACK_DTYPE in order, arrays flattened).  Entries past a frame's count hold no result and are
+    written as zeros (-1 for ids), so equal inputs give equal files.  If the batch would exceed `limit` bytes, a fixed, seeded
+    sample of its frames is written instead; `frame_index` lists the frames kept."""
+    B = int(np.asarray(r.counts).shape[0])
+    keep = np.arange(B)
+    arrays = _step_arrays(r, keep)
+    size = sum(a.nbytes for a in arrays.values())
+    while size > limit and len(keep) > 1:
+        n = max(1, min(len(keep) - 1, len(keep) * limit // size))
+        keep = np.sort(np.random.default_rng(0).choice(B, n, replace=False))
+        arrays = _step_arrays(r, keep)
+        size = sum(a.nbytes for a in arrays.values())
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return arrays
 
 
 class ClockSampler:
@@ -239,6 +288,8 @@ def run_b200(args):
             copy_ev[slot].record(copy_stream)
 
     def run_steps(n, first, on_device):
+        """n steps from pool batch `first` on; returns the result of the last one"""
+        last = None
         if not on_device:
             upload(0, first % pool_batches)
         for i in range(n):
@@ -250,10 +301,14 @@ def run_b200(args):
                 if i + 1 < n:
                     upload((i + 1) % NS, (first + i + 1) % pool_batches)
                 ptr = stage[i % NS].data_ptr()
-            gather(pipe.step_pipelined(ptr, True, (B, FRAME_H, FRAME_W)))
+            r = pipe.step_pipelined(ptr, True, (B, FRAME_H, FRAME_W))
+            gather(r)
+            last = r if r is not None else last
         for r in pipe.flush():
             gather(r)
+            last = r
         final_gather()
+        return last
 
     sampler = ClockSampler(local)
 
@@ -264,7 +319,7 @@ def run_b200(args):
         w0 = time.time()
         pipe.yolo.event_record(0)
         t0 = time.perf_counter()
-        run_steps(K, Wm, on_device)
+        last = run_steps(K, Wm, on_device)
         pipe.ufld.event_record(1)
         pipe.yolo.event_record(1)
         torch.cuda.synchronize()
@@ -279,7 +334,7 @@ def run_b200(args):
             t = torch.tensor([ms], dtype=torch.float64, device=f"cuda:{local}")
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
-        return ms, launches, clocks
+        return ms, launches, clocks, last
 
     if args.profile_steps:
         # profiler target (ncu --profile-from-start off): warm up (autotune, graph capture), then expose N steps; no numbers printed
@@ -292,9 +347,11 @@ def run_b200(args):
         pipe.close()
         return
     sampler.start()
-    ms_dev, launches, clocks = timed(True)
-    ms_e2e, _, clocks_e2e = timed(False)
+    ms_dev, launches, clocks, _ = timed(True)
+    ms_e2e, _, clocks_e2e, last = timed(False)
     sampler.close()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(last, args.dump_outputs)
 
     result = None
     if rank == 0:
@@ -458,9 +515,7 @@ def run_reference(args):
     path = CpuReferencePath(plans)
     per_step = args.ref_frames
     K, Wm = args.steps, max(args.warmup, 1)
-    # bound the run to a few minutes: ~1 s of CPU per frame
-    K = min(K, max(3, int(150 / max(per_step, 1))))
-    Wm = min(Wm, 2)
+    Wm = min(Wm, 2)                         # at most two warm-up steps: ~1 s of CPU per frame
     imgs = synth_stream(1000, per_step * 4)
     for i in range(Wm):
         for f in range(per_step):
@@ -499,7 +554,22 @@ def main():
     ap.add_argument("--ref-frames", type=int, default=2, help="frames per step of the --impl reference arm")
     ap.add_argument("--watchdog", type=int, default=int(os.environ.get("ADAS_B200_WATCHDOG", "1500")),
                     help="seconds after which a stuck run dumps every thread's stack to stderr and exits non-zero (0 disables)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (detections, lanes, tracks of rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.profile_steps):
+        ap.error("--dump-outputs needs the timed steps of --impl b200")
+    if not os.environ.get("ADAS_B200_PLAN_CACHE"):
+        # the plans are rebuilt from their seeds on every run anyway: write their files to a private temporary directory that is
+        # removed at exit, so a run needs no writable home directory and leaves nothing behind
+        import atexit
+        import shutil
+        import tempfile
+        tmp = tempfile.mkdtemp(prefix="adas_b200_bench_")
+        atexit.register(shutil.rmtree, tmp, True)
+        os.environ["ADAS_B200_PLAN_CACHE"] = tmp
     if args.watchdog > 0:
         import faulthandler
         faulthandler.dump_traceback_later(args.watchdog, exit=True, file=sys.stderr)      # a hang must end loudly, with evidence
