@@ -231,6 +231,8 @@ def test_stem_repack_7x7s2(tmp_path, impl):
 
 @pytest.mark.parametrize("impl", [1, 0])
 def test_fc_swap_ab(tmp_path, impl):
+    """FC layers (swap-AB plan ops) with at most 48 MiB of fp16 weights: impl 0 runs them as fc_stream_kernel, impl 1 through the
+    SIMT validation kernel.  The tcgen05 swap-AB GEMM, which takes the larger FCs, is checked in test_gpu_lane_head.py."""
     rng = np.random.default_rng(3)
     for (B, K, N, act) in ((3, 4992, 2048, 2), (8, 2048, 9128, 0), (1, 256, 136, 0)):
         pb = plan.PlanBuilder(plan.MODEL_UFLDV2, 3, 8, 8)
@@ -247,6 +249,8 @@ def test_fc_swap_ab(tmp_path, impl):
         for _ in range(3):
             eng.run(B)
         got = eng.read_buffer(out, B).astype(np.float32)
+        if impl == 0:
+            assert "fc_stream" in eng.time_step(B, 0, 1)[2]
         ref = x.astype(np.float32) @ w.astype(np.float16).astype(np.float32).T + b
         if act == 2:
             ref = np.maximum(ref, 0)

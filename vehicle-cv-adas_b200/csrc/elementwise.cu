@@ -179,36 +179,55 @@ int launch_upsample2x(const __half* in, int in_ld, int B, int H, int W, int C, _
 }
 
 // ---- LayerNorm over a feature row (one CTA per row), fp32 statistics ------------------------------
+// Block-wide sums of a and b (fixed order: lanes, then warps), returned to every thread.  The leading barrier lets the kernel call
+// it twice on the same shared buffer: nobody overwrites it before every thread has read the previous result.
+__device__ __forceinline__ void block_sum2(float& a, float& b, float (*red)[32]) {
+    for (int o = 16; o > 0; o >>= 1) {
+        a += __shfl_xor_sync(0xffffffffu, a, o);
+        b += __shfl_xor_sync(0xffffffffu, b, o);
+    }
+    const int w = threadIdx.x >> 5, l = threadIdx.x & 31;
+    __syncthreads();
+    if (l == 0) { red[0][w] = a; red[1][w] = b; }
+    __syncthreads();
+    if (w == 0) {
+        a = (l < (int)(blockDim.x >> 5)) ? red[0][l] : 0.f;
+        b = (l < (int)(blockDim.x >> 5)) ? red[1][l] : 0.f;
+        for (int o = 16; o > 0; o >>= 1) {
+            a += __shfl_xor_sync(0xffffffffu, a, o);
+            b += __shfl_xor_sync(0xffffffffu, b, o);
+        }
+        if (l == 0) { red[0][0] = a; red[1][0] = b; }
+    }
+    __syncthreads();
+    a = red[0][0];
+    b = red[1][0];
+}
+
+// Two passes over the row (the UFLD slab is 10 KB, re-read from L1): the mean, then the squared deviations from it.  The one-pass
+// E[x^2] - mean^2 loses the variance to cancellation once |mean| / std nears 100 (pool-conv features with a large bias).  The
+// d_len - d_norm structural entries of the slab are zeros (plan.h), so the second pass skips zero entries and adds the real ones
+// among them back as (Dn - nonzeros) * mean^2.
 __global__ void layernorm_kernel(const __half* __restrict__ in, int in_ld, int D, int Dn, const float* __restrict__ gamma,
                                  const float* __restrict__ beta, float eps, __half* __restrict__ out, int out_ld) {
     const int row = blockIdx.x;
     const __half* x = in + (size_t)row * in_ld;
     __shared__ float red[2][32];
-    float s = 0.f, ss = 0.f;
+    float s = 0.f, unused = 0.f;
+    for (int i = threadIdx.x; i < D; i += blockDim.x) s += __half2float(x[i]);
+    block_sum2(s, unused, red);
+    const float mean = s / Dn;
+    float q = 0.f, nz = 0.f;
     for (int i = threadIdx.x; i < D; i += blockDim.x) {
         const float v = __half2float(x[i]);
-        s += v;
-        ss += v * v;
-    }
-    for (int o = 16; o > 0; o >>= 1) {
-        s += __shfl_xor_sync(0xffffffffu, s, o);
-        ss += __shfl_xor_sync(0xffffffffu, ss, o);
-    }
-    const int w = threadIdx.x >> 5, l = threadIdx.x & 31;
-    if (l == 0) { red[0][w] = s; red[1][w] = ss; }
-    __syncthreads();
-    if (w == 0) {
-        s = (l < (int)(blockDim.x >> 5)) ? red[0][l] : 0.f;
-        ss = (l < (int)(blockDim.x >> 5)) ? red[1][l] : 0.f;
-        for (int o = 16; o > 0; o >>= 1) {
-            s += __shfl_xor_sync(0xffffffffu, s, o);
-            ss += __shfl_xor_sync(0xffffffffu, ss, o);
+        if (v != 0.f) {
+            const float d = v - mean;
+            q += d * d;
+            nz += 1.f;
         }
-        if (l == 0) { red[0][0] = s; red[1][0] = ss; }
     }
-    __syncthreads();
-    const float mean = red[0][0] / Dn;
-    const float var = fmaxf(red[1][0] / Dn - mean * mean, 0.f);
+    block_sum2(q, nz, red);
+    const float var = fmaxf((q + ((float)Dn - nz) * mean * mean) / Dn, 0.f);
     const float rstd = rsqrtf(var + eps);
     for (int i = threadIdx.x; i < D; i += blockDim.x) {
         const float v = (__half2float(x[i]) - mean) * rstd * gamma[i] + beta[i];
