@@ -264,6 +264,11 @@ int adas_engine_time_ops(adas_engine* e, int batch, unsigned type_mask, int iter
  * description of the GEMM shape / tile choice (empty for non-GEMM steps). */
 int adas_engine_num_steps(adas_engine* e, int batch, int* n);
 int adas_engine_time_step(adas_engine* e, int batch, int step, int iters, float* ms_per_iter, int* op_type, char* desc, int desc_cap);
+/* adas_engine_step_tiles: the (BN, MT) tiles the tcgen05 GEMM of launch `step` could have run with at `batch` -- every candidate
+ * the program build prepared and launched without error while timing, in cost-model order (with ADAS_B200_AUTOTUNE=0 or a
+ * plan-forced tile: the one tile in use).  *chosen = index of the tile the program runs (-1 when *n = 0).  Writes at most `cap` entries; *n is
+ * the full count, 0 for a step that is not a tcgen05 GEMM (FC weight stream, im2col, stem conv, SIMT kernel, chain steps). */
+int adas_engine_step_tiles(adas_engine* e, int batch, int step, int cap, int* bn, int* mt, int* n, int* chosen);
 
 /* ---- optional multi-GPU gather -------------------------------------------------------------
  * (no reference counterpart: the reference is single-GPU, SURVEY 8e; BASELINE configs[4] asks for an NCCL gather of boxes.)

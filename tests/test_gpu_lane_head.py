@@ -16,9 +16,9 @@ from scipy.special import expit
 import synth
 import adas_b200  # noqa: F401
 from adas_b200 import _capi, plan
-from gpu_util import cached_plan, to_padded
+from gpu_util import U16, U32, cached_plan, to_padded
+from gpu_util import check as _check
 
-U32, U16 = 2.0 ** -24, 2.0 ** -11      # unit roundoff of fp32 and of fp16
 FC_STREAM_MAX_BYTES = 48 << 20          # engine.cu: an FC with at most this many bytes of fp16 weights runs as fc_stream_kernel
 RELU, SILU, NONE = plan.ACT_RELU, plan.ACT_SILU, plan.ACT_NONE
 
@@ -47,16 +47,6 @@ def fc_reference(x16, w16, b, act, chunk=8192):
         ref[:, n0:n0 + chunk] = x @ w.T + b[n0:n0 + chunk]
         mag[:, n0:n0 + chunk] = ax @ np.abs(w).T
     return _act64(ref, act), mag
-
-
-def _check(got, ref, tol, what):
-    err = np.abs(got.astype(np.float64) - ref)
-    bad = ~(err <= tol)                    # a NaN fails too
-    if bad.any():
-        i = np.unravel_index(np.argmax(bad), bad.shape)
-        raise AssertionError(f"{what}: {int(bad.sum())} of {bad.size} elements outside the bound; first at {i}: got {got[i]}, "
-                             f"reference {ref[i]:.7g}, bound {tol[i]:.3g}")
-    return float((err / tol).max())
 
 
 def check_fc(got, ref, mag, K, f16_out, what="fc"):

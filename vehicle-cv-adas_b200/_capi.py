@@ -23,7 +23,7 @@ SYMBOLS = [
     "adas_engine_infer", "adas_engine_infer_dev", "adas_yolo_detect", "adas_yolo_postprocess", "adas_yolo_preprocess",
     "adas_ufld_detect", "adas_ufld_postprocess", "adas_ufld_v1_postprocess", "adas_lane_geometry", "adas_ufld_lane_geometry", "adas_warp_perspective", "adas_engine_warp_perspective", "adas_ufld_preprocess", "adas_iou_cost", "adas_lap", "adas_associate",
     "adas_engine_stream", "adas_engine_num_buffers", "adas_engine_buffer_info", "adas_engine_write_buffer", "adas_engine_read_buffer",
-    "adas_engine_run", "adas_engine_event_record", "adas_event_elapsed_ms", "adas_engine_time_ops", "adas_engine_num_steps", "adas_engine_time_step", "adas_detect_pair",
+    "adas_engine_run", "adas_engine_event_record", "adas_event_elapsed_ms", "adas_engine_time_ops", "adas_engine_num_steps", "adas_engine_time_step", "adas_engine_step_tiles", "adas_detect_pair",
     "adas_comm_unique_id", "adas_comm_create", "adas_comm_destroy", "adas_comm_all_gather", "adas_comm_sync", "adas_comm_read", "adas_comm_info",
     "adas_tracker_create", "adas_tracker_destroy", "adas_tracker_reset", "adas_tracker_update", "adas_tracker_update_batch", "adas_tracker_get", "adas_tracker_count", "adas_tracker_stats",
 ]
@@ -214,6 +214,15 @@ class Engine:
         buf = C.create_string_buffer(256)
         check(lib().adas_engine_time_step(self._h, batch, step, iters, C.byref(ms), C.byref(t), buf, 256))
         return float(ms.value), int(t.value), buf.value.decode()
+
+    def step_tiles(self, batch: int, step: int):
+        """([(BN, MT), ...], chosen): the tiles the tcgen05 GEMM of launch `step` could have run with at `batch`, in cost-model order,
+        and the index of the one it runs.  ([], -1) for a step that is not a tcgen05 GEMM."""
+        bn, mt = (C.c_int * 16)(), (C.c_int * 16)()
+        n, chosen = C.c_int(), C.c_int()
+        check(lib().adas_engine_step_tiles(self._h, batch, step, 16, bn, mt, C.byref(n), C.byref(chosen)))
+        assert n.value <= 16
+        return [(int(bn[i]), int(mt[i])) for i in range(n.value)], int(chosen.value)
 
     # engine_inference: fp32 NCHW host -> list of fp32 host arrays
     def infer(self, x: np.ndarray):

@@ -43,6 +43,8 @@ struct Program {   // launch list for one batch size
     std::vector<std::function<int(cudaStream_t)>> steps;
     std::vector<uint32_t> step_type;
     std::vector<std::string> step_desc;   // human-readable shape / tile choice per step (adas_engine_step_desc)
+    std::vector<std::vector<std::pair<int, int>>> step_tiles;   // (BN, MT) tiles a tcgen05 GEMM step could run with (adas_engine_step_tiles)
+    std::vector<int> step_chosen;                               // index into step_tiles of the tile the step runs
     cudaGraphExec_t graph = nullptr;
     int runs = 0;
     int n_launch() const { int n = 0; for (uint32_t t : step_type) n += (t != 31); return n; }   // steps folded into a chain launch do not launch
@@ -222,6 +224,7 @@ static int build_chains(adas_engine* e, Program* prog, std::vector<GemmRec>& rec
                 prog->step_desc.resize(prog->steps.size());
                 prog->step_desc[recs[i].step] = d;
                 prog->steps[recs[i].step] = [keep](cudaStream_t st) { return gemm_chain_run(keep.get(), st); };
+                for (size_t k = i; k <= j; ++k) prog->step_tiles[recs[k].step].clear();      // no longer a per-layer tcgen05 GEMM launch
                 for (size_t k = i + 1; k <= j; ++k) {
                     prog->steps[recs[k].step] = [](cudaStream_t) { return 0; };   // folded into the chain launch above
                     prog->step_type[recs[k].step] = 31;
@@ -342,6 +345,8 @@ static int build_program(adas_engine* e, int batch, Program* prog) {
                 if (e->conv_impl == 0) {
                     // ---- product path: gemm_v3.cu ----
                     void* opaque = nullptr;
+                    std::vector<std::pair<int, int>> tiles;       // every tile that was prepared and launched (adas_engine_step_tiles)
+                    int chosen = 0;
                     const uint64_t a_Wp = (uint64_t)ab.W + 2, a_Hp = (uint64_t)ab.H + 2, a_ldC = (uint64_t)ab.C;
                     std::function<int(const GemmParams&, void**)> prep = [=](const GemmParams& gc, void** out) -> int {
                         if (s2) return gemm_v3_prepare_s2(gc, aptr, (uint64_t)Kc, a_Wp, a_Hp, (uint64_t)batch, a_ldC, opB, b_inner, b_rows_u, b_stride, out);
@@ -360,7 +365,9 @@ static int build_program(adas_engine* e, int batch, Program* prog) {
                             gc.BN = cBN[ci]; gc.mt_hint = cMT[ci];
                             void* cand = nullptr;
                             if (prep(gc, &cand)) continue;
-                            if (nc == 1) { opaque = cand; break; }
+                            std::pair<int, int> tile;
+                            gemm_v3_tile_of(cand, &tile.first, &tile.second);
+                            if (nc == 1) { opaque = cand; tiles.push_back(tile); break; }
                             int rc = gemm_v3_run(cand, e->stream);
                             if (!rc) {
                                 cudaEventRecord(ev0, e->stream);
@@ -373,13 +380,16 @@ static int build_program(adas_engine* e, int batch, Program* prog) {
                             static const bool at_log = getenv("ADAS_B200_AT_LOG") != nullptr;
                             if (at_log) fprintf(stderr, "[autotune] op %zu M=%d N=%d K=%d taps=%d s2=%d BN=%d mt=%d : %.1f us\n", oi, g.M, g.N, Kc * ntaps, ntaps, s2,
                                                 gc.BN, gc.mt_hint, rc ? -1.0 : ms * 1000.0 / 4.0);
-                            if (!rc && ms < best_ms) { best_ms = ms; if (opaque) gemm_v3_free(opaque); opaque = cand; }
+                            if (!rc) tiles.push_back(tile);
+                            if (!rc && ms < best_ms) { best_ms = ms; if (opaque) gemm_v3_free(opaque); opaque = cand; chosen = (int)tiles.size() - 1; }
                             else gemm_v3_free(cand);
                         }
                         if (ev0) { cudaEventDestroy(ev0); cudaEventDestroy(ev1); }
                         ADAS_CHECK(opaque != nullptr, "op %zu: no GEMM tile configuration could be launched (%s)", oi, g_err);
                     } else {
                         if (prep(g, &opaque)) return 1;
+                        tiles.emplace_back();
+                        gemm_v3_tile_of(opaque, &tiles[0].first, &tiles[0].second);
                     }
                     std::shared_ptr<void> keep(opaque, gemm_v3_free);
                     {
@@ -387,6 +397,10 @@ static int build_program(adas_engine* e, int batch, Program* prog) {
                         gemm_v3_describe(opaque, d, sizeof(d));
                         prog->step_desc.resize(prog->step_type.size());
                         prog->step_desc.back() = d;
+                        prog->step_tiles.resize(prog->step_type.size());
+                        prog->step_tiles.back() = tiles;
+                        prog->step_chosen.resize(prog->step_type.size());
+                        prog->step_chosen.back() = chosen;
                     }
                     {
                         GemmRec rec;
@@ -484,6 +498,8 @@ static int build_program(adas_engine* e, int batch, Program* prog) {
         }
     }
     prog->step_desc.resize(prog->steps.size());
+    prog->step_tiles.resize(prog->steps.size());
+    prog->step_chosen.resize(prog->steps.size());
     return build_chains(e, prog, recs);
 }
 
@@ -1386,6 +1402,23 @@ int adas_engine_num_steps(adas_engine* e, int batch, int* n) {
         it = e->programs.emplace(batch, std::move(prog)).first;
     }
     *n = (int)it->second.steps.size();
+    return 0;
+}
+int adas_engine_step_tiles(adas_engine* e, int batch, int step, int cap, int* bn, int* mt, int* n, int* chosen) {
+    ADAS_CHECK(e != nullptr && batch >= 1 && batch <= e->max_batch && cap >= 0 && n != nullptr && chosen != nullptr, "bad arguments");
+    ADAS_CUDA(cudaSetDevice(e->device));
+    auto it = e->programs.find(batch);
+    if (it == e->programs.end()) {
+        Program prog;
+        if (build_program(e, batch, &prog)) return 1;
+        it = e->programs.emplace(batch, std::move(prog)).first;
+    }
+    const Program& pg = it->second;
+    ADAS_CHECK(step >= 0 && step < (int)pg.steps.size(), "step %d outside [0, %d)", step, (int)pg.steps.size());
+    const std::vector<std::pair<int, int>>& t = pg.step_tiles[step];
+    for (int i = 0; i < (int)t.size() && i < cap; ++i) { bn[i] = t[i].first; mt[i] = t[i].second; }
+    *n = (int)t.size();
+    *chosen = t.empty() ? -1 : pg.step_chosen[step];
     return 0;
 }
 

@@ -295,10 +295,11 @@ class PlanBuilder:
         self._op(OP_STEMCONV, [x.buf, w_t, bias_t, cout, k, pad, act, out.buf, out.coff])
         return View(out.buf, out.coff, cout, out.H, out.W)
 
-    def stem7x7s2(self, x: View, w: np.ndarray, b: np.ndarray, act: int) -> View:
+    def stem7x7s2(self, x: View, w: np.ndarray, b: np.ndarray, act: int, tile: Optional[Tuple[int, int]] = None) -> View:
         """7x7 stride-2 pad-3 conv on the C=4 image without a patch matrix: the image is re-laid out once as
         Q[j][xo][p*32 + kx*4 + c] = img[2j-1+p][2xo+kx-3][c] (row PAIRS x the 7 horizontal taps = 64 channels) on the
-        OUTPUT's padded grid, which turns the conv into 4 vertically shifted GEMM taps of K = 64 (rows yo-1 .. yo+2)."""
+        OUTPUT's padded grid, which turns the conv into 4 vertically shifted GEMM taps of K = 64 (rows yo-1 .. yo+2).
+        tile = (BN, MT) forces the GEMM's tile shape, as in conv()."""
         cout, cin_real = int(w.shape[0]), int(w.shape[1])
         assert w.shape[2:] == (7, 7) and x.C == 4 and cin_real <= 4 and x.H % 2 == 0 and x.W % 2 == 0
         Ho, Wo = x.H // 2, x.W // 2
@@ -315,7 +316,8 @@ class PlanBuilder:
         w_t = self.tensor(wq.reshape(cout, 256).astype(np.float16))
         bias_t = self.tensor(b.astype(np.float32))
         # ntaps = 4 selects the vertical tap table (row shifts -2, -1, 0, +1 padded rows)
-        self._op(OP_GEMM, [q.buf, 0, 64, 4, w_t, bias_t, cout, act, -1, 0, 0, out.buf, 0, 1, 0, 0, 0])
+        bn, mt = tile if tile is not None else (0, 0)
+        self._op(OP_GEMM, [q.buf, 0, 64, 4, w_t, bias_t, cout, act, -1, 0, 0, out.buf, 0, 1, 0, bn, 0, mt])
         return View(out.buf, 0, cout, Ho, Wo)
 
     def maxpool(self, x: View, k: int, s: int, p: int, out: Optional[View] = None) -> View:
